@@ -60,7 +60,15 @@ def parse_args():
     ap.add_argument("--no-secondary", action="store_true", help="skip the quick batch-1/256, A2, LSTM, a2_max lines")
     ap.add_argument("--no-gather", action="store_true",
                     help="N > 1: skip the second timed pass that all-gathers every step's outputs over NCCL")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/y.npy (DIR/y_rank<r>.npy at N > 1), float32, "
+                         "streams x frames; above 64 MB in all, a fixed seeded choice of streams in ascending order")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
+    if args.dump_outputs and args.steps < 1:
+        ap.error("--dump-outputs writes the outputs of the last timed step: --steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -230,7 +238,7 @@ def cpu_arms(nam: dict, fast_tanh: bool, frames: int, streams_per_thread: int) -
         if r is not None:
             out["reference"] = {"value": r[0], "seconds": r[1], "cores": cores, "streams": streams,
                                 "flags": f"g++ -Ofast -march={'x86-64-v4' if r[2] == 'fast512' else 'x86-64-v3'} "
-                                         "(tools/CMakeLists.txt:106), unmodified /root/reference/NAM sources, Eigen stand-in"}
+                                         "(tools/CMakeLists.txt:106), the unmodified reference NAM sources, Eigen stand-in"}
     except Exception as exc:  # the reference build is optional on the box
         out["reference_error"] = str(exc)[:200]
     kind = "reference" if out.get("reference", {}).get("value", 0.0) > v else "port"
@@ -346,6 +354,24 @@ def workload_config(args) -> dict:
     }
 
 
+DUMP_BYTES = 64 * 10**6  # --dump-outputs: at most this much in all, over every rank
+
+
+def dump_outputs(out_dir: str, y, rank: int, world: int) -> None:
+    """y (streams x frames, float32 on the device) -> out_dir/y.npy.  Where all ranks' outputs would exceed DUMP_BYTES,
+    each rank keeps the same seeded choice of streams, so two runs with the same arguments write the same streams."""
+    import torch
+
+    streams, frames = y.shape
+    keep = min(streams, DUMP_BYTES // (world * frames * y.element_size()))
+    if keep < 1:
+        raise SystemExit(f"bench.py: --dump-outputs: one stream of {frames} frames exceeds {DUMP_BYTES} bytes")
+    rows = np.arange(streams) if keep == streams else np.sort(np.random.default_rng(0).choice(streams, keep, replace=False))
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / ("y.npy" if world == 1 else f"y_rank{rank}.npy"), y[torch.from_numpy(rows).to(y.device)].cpu().numpy())
+
+
 def run_b200(args) -> None:
     import torch
 
@@ -411,6 +437,8 @@ def run_b200(args) -> None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total_ms_max = float(t.item())
     value = world * B * n * args.steps / (total_ms_max * 1e-3) / 1e6
+    if args.dump_outputs:  # before the passes below write y_dev again
+        dump_outputs(args.dump_outputs, y_dev, rank, world)
 
     # ---- end to end through the host API ----
     e2e = None

@@ -1,6 +1,6 @@
 """ctypes front-end for oracle/_ref/libnam_ref.so: the UNMODIFIED reference (NeuralAmpModelerCore) compiled from
-its own sources against oracle/eigen_shim (recipe: `make -C oracle ref`, only where /root/reference is mounted;
-the .so is git-ignored but travels to the GPU box).
+its own sources against oracle/eigen_shim (recipe: `make -C oracle ref`, run by build() where the reference checkout
+-- oracle/Makefile's REF, or the NAM_REFERENCE environment variable -- is readable; the .so is git-ignored).
 
 TEST INFRASTRUCTURE ONLY, like the rest of oracle/: it pins the C restatement (nam_oracle.c) and the CUDA path
 against the reference's own code at whole-model level.  Nothing in the product imports this module.
@@ -18,7 +18,6 @@ import numpy as np
 
 HERE = Path(__file__).resolve().parent
 REF_DIR = HERE / "_ref"
-REFERENCE_TREE = Path("/root/reference")
 _LIBS: dict[str, C.CDLL] = {}
 
 
@@ -32,11 +31,24 @@ def available(variant: str = "default") -> bool:
     return lib_path(variant).exists()
 
 
+def reference_tree() -> Path | None:
+    """The reference checkout: NAM_REFERENCE if set, else oracle/Makefile's REF default; None where it is absent or not
+    readable by this user."""
+    tree = os.environ.get("NAM_REFERENCE") or subprocess.run(
+        ["make", "-s", "--no-print-directory", "-C", str(HERE), "ref_tree"], capture_output=True, text=True,
+        check=True).stdout.strip()
+    try:
+        return Path(tree) if (Path(tree) / "NAM" / "dsp.cpp").is_file() else None
+    except OSError:  # a directory on the way this user may not enter
+        return None
+
+
 def build(force: bool = False) -> bool:
-    """Compile the reference where its sources are mounted; returns False (and builds nothing) elsewhere."""
-    if not (REFERENCE_TREE / "NAM" / "dsp.cpp").exists():
+    """Compile the reference and its tools from reference_tree(); returns False (and builds nothing) without one."""
+    tree = reference_tree()
+    if tree is None:
         return False
-    cmd = ["make", "-C", str(HERE), "ref"] + (["-B"] if force else [])
+    cmd = ["make", "-C", str(HERE), "ref", "ref_tools", f"REF={tree}"] + (["-B"] if force else [])
     subprocess.run(cmd, check=True, capture_output=True)
     return True
 

@@ -1,7 +1,8 @@
-"""Drop-in proof on the GPU box: the reference's OWN tools (tools/benchmodel.cpp, tools/render.cpp,
-tools/loadmodel.cpp), compiled unchanged against include/NAM/*.h + libnam_b200.so by tools/build_tools.sh
-in the build container, run here and are checked against the CPU oracle.  Also the repo's own C++ host
-tool over the C ABI.  Skipped when the binaries were not built (no reference tree at build time)."""
+"""Drop-in proof on the GPU: the reference's OWN tools (tools/benchmodel.cpp, tools/render.cpp,
+tools/loadmodel.cpp), compiled unchanged against include/NAM/*.h + libnam_b200.so into oracle/_ref/tools/ by
+`make -C oracle ref_tools` (build() runs it where the reference checkout is readable), run here and are
+checked against the CPU oracle.  Also the repo's own C++ host tool over the C ABI.  The reference's tools are skipped
+where they were not built: their sources are not part of this repository."""
 import json
 import struct
 import subprocess
@@ -15,7 +16,7 @@ from tests import nam_fixtures as fx
 
 pytestmark = pytest.mark.gpu
 ROOT = Path(__file__).resolve().parents[1]
-REF_TOOLS = ROOT / "build" / "ref_tools"
+REF_TOOLS = ROOT / "oracle" / "_ref" / "tools"
 
 
 def _write_nam(tmp_path, name):

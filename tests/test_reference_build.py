@@ -1,17 +1,16 @@
-"""Whole-model pin of the oracle against THE REFERENCE ITSELF: oracle/_ref/libnam_ref.so is the unmodified
-NeuralAmpModelerCore source tree compiled against a stand-in for its missing Eigen submodule
-(oracle/eigen_shim, recipe `make -C oracle ref`).  The reference's own tests hold no whole-model vectors
-(SURVEY.md 8c), so this is what turns the oracle's model-level reading of the reference -- weight order, prewarm,
-head_scale, condition_dsp, containers, the A2 fast path -- from "restated" into "checked".
+"""Whole-model pin of the oracle against THE REFERENCE ITSELF: the unmodified NeuralAmpModelerCore source tree compiled
+against a stand-in for its missing Eigen submodule (oracle/eigen_shim, recipe `make -C oracle ref`), whose outputs
+are recorded in tests/golden/reference_outputs.npz (tests/reference_outputs.py).  The reference's own tests hold no
+whole-model vectors (SURVEY.md 8c), so this is what turns the oracle's model-level reading of the reference -- weight
+order, prewarm, head_scale, condition_dsp, containers, the A2 fast path -- from "restated" into "checked".
 
-Runs on CPU.  Skipped where the library was not built (no reference tree at build time)."""
+Runs on CPU."""
 import numpy as np
 import pytest
 
 from oracle import oracle, ref
 from tests import nam_fixtures as fx
-
-pytestmark = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libnam_ref.so not built (no /root/reference)")
+from tests import reference_outputs as R
 
 # two independent fp32 implementations (different summation order inside the matrix products): the reference's
 # authors accept 5e-5 between two of their own (tools/test/test_a2_fast.cpp:296-298); measured here <= 3e-6
@@ -24,20 +23,24 @@ def _rel(err, y):
     return err / max(1.0, float(np.max(np.abs(y))))
 
 
+def _oracle(nam, x, block=64, fast=False):
+    m = oracle.OracleModel.from_dict(nam, fast_tanh=fast)
+    m.reset(48000.0, block)
+    return m.run(x, block)
+
+
 @pytest.mark.parametrize("name", MODELS)
 @pytest.mark.parametrize("fast", [False, True], ids=["exact_tanh", "fast_tanh"])
 def test_oracle_matches_the_reference_build(name, fast):
     nam = fx.load_model(name)
     x = fx.input_wav()[43000:53000]  # 5,000 frames of silence, then the 220 Hz sine
-    r = ref.ReferenceModel.from_dict(nam, fast_tanh=fast)
-    r.reset(48000.0, 64)
+    want = R.expected(f"wav/{name}/{R.regime(fast)}")
     m = oracle.OracleModel.from_dict(nam, fast_tanh=fast)
     m.reset(48000.0, 64)
-    assert r.prewarm_samples == m.prewarm_samples
-    yr, yo = r.run(x, 64), m.run(x, 64)
+    assert want["prewarm_samples"] == m.prewarm_samples
+    yr, yo = want["y"], R.sample(m.run(x, 64))
     err = float(np.max(np.abs(yr - yo)))
     assert _rel(err, yr) <= TOL, f"{name}: max|reference - oracle| = {err:.3e} (max|y| {np.max(np.abs(yr)):.3f})"
-    r.close()
 
 
 @pytest.mark.parametrize("name", ["wavenet_a1_standard", "a2_full", "lstm"])
@@ -47,72 +50,45 @@ def test_block_size_protocols_agree(name):
     nam = fx.load_model(name)
     x = fx.synthetic_batch(1, 3000, seed=17)[0]
     for block in (64, 1000):
-        r = ref.ReferenceModel.from_dict(nam)
-        r.reset(48000.0, block)
-        m = oracle.OracleModel.from_dict(nam)
-        m.reset(48000.0, block)
-        yr, yo = r.run(x, block), m.run(x, block)
+        yr = R.expected(f"blocks/{name}/{block}")["y"]
+        yo = R.sample(_oracle(nam, x, block))
         assert _rel(float(np.max(np.abs(yr - yo))), yr) <= TOL, f"{name} block {block}"
-        r.close()
 
 
 def test_golden_vectors_were_not_a_misreading():
     """The committed oracle vectors (tests/golden/oracle_outputs.npz) against the reference build, full 2 s."""
-    x = fx.input_wav()
     for name in ("wavenet", "wavenet_a1_standard", "a2_full"):
         gold = fx.oracle_golden(name, "exact")
-        r = ref.ReferenceModel.from_dict(fx.load_model(name))
-        r.reset(48000.0, 64)
-        y = r.run(x, 64)
-        r.close()
-        for key, val in fx.decimate(y).items():
-            assert np.max(np.abs(val - gold[key])) <= TOL, f"{name} {key}"
+        for key, val in R.expected(f"full_input/{name}").items():
+            assert np.max(np.abs(val - R.sample(gold[key]))) <= TOL, f"{name} {key}"
 
 
 def test_a2_fast_path_and_generic_path_of_the_reference():
     """The default reference build routes A2 shapes to A2FastModel (model.cpp:1317-1320); the second build has the
     fast path compiled out.  Both must agree with the oracle (and so with each other)."""
-    if not ref.available("generic"):
-        pytest.skip("generic variant not built")
     x = fx.synthetic_batch(1, 4000, seed=3)[0]
     for name in ("a2_lite", "a2_full"):
-        nam = fx.load_model(name)
-        m = oracle.OracleModel.from_dict(nam)
-        m.reset(48000.0, 64)
-        yo = m.run(x, 64)
+        yo = R.sample(_oracle(fx.load_model(name), x))
         for variant in ("default", "generic"):
-            r = ref.ReferenceModel.from_dict(nam, variant=variant)
-            r.reset(48000.0, 64)
-            err = float(np.max(np.abs(r.run(x, 64) - yo)))
+            err = float(np.max(np.abs(R.expected(f"a2_variants/{name}/{variant}")["y"] - yo)))
             assert err <= TOL, f"{name} {variant}: {err:.3e}"
-            r.close()
 
 
 def test_slimmable_container_semantics():
     """ContainerModel (container.cpp): full size by default; SetSlimmableSize before or after Reset; the newly
     active sub-model starts from its own prewarmed state."""
     lite, full = fx.load_model("a2_lite"), fx.load_model("a2_full")
-    cont = fx.make_container([(0.5, lite), (1.0, full)])
     x = fx.synthetic_batch(1, 2000, seed=9)[0]
+    want = R.expected("container_semantics")
 
     def orc(nam, sig):
-        m = oracle.OracleModel.from_dict(nam)
-        m.reset(48000.0, 64)
-        return m.run(sig, 64)
+        return R.sample(_oracle(nam, sig))
 
-    r = ref.ReferenceModel.from_dict(cont)
-    r.reset(48000.0, 64)
-    assert np.max(np.abs(r.run(x[:1000], 64) - orc(full, x[:1000]))) <= TOL
-    r.set_slimmable_size(0.2)
-    assert np.max(np.abs(r.run(x, 64) - orc(lite, x))) <= TOL
-    r.set_slimmable_size(0.5)  # 0.5 is not < 0.5 -> full again, freshly reset
-    assert np.max(np.abs(r.run(x[:640], 64) - orc(full, x[:640]))) <= TOL
-    r.close()
-    r = ref.ReferenceModel.from_dict(cont)
-    r.set_slimmable_size(0.1)  # before the first Reset (tools/render.cpp:117-126 order)
-    r.reset(48000.0, 64)
-    assert np.max(np.abs(r.run(x, 64) - orc(lite, x))) <= TOL
-    r.close()
+    assert np.max(np.abs(want["full_first"] - orc(full, x[:1000]))) <= TOL
+    assert np.max(np.abs(want["small"] - orc(lite, x))) <= TOL  # SetSlimmableSize(0.2)
+    assert np.max(np.abs(want["full_again"] - orc(full, x[:640]))) <= TOL  # 0.5 is not < 0.5 -> full again, freshly reset
+    # SetSlimmableSize(0.1) before the first Reset (tools/render.cpp:117-126 order)
+    assert np.max(np.abs(want["small_before_reset"] - orc(lite, x))) <= TOL
 
 
 def _multichannel_models():
@@ -138,23 +114,26 @@ def _multichannel_models():
         yield f"lstm {ci} in / {co} out", rnd(nam, ci * 10 + co)
 
 
+def _planar_against_the_reference(nam, fast, n, block, seed, key, label=""):
+    """Multi-channel DSP::process calls of `block` frames on synthetic input, the oracle against the recorded run."""
+    want = R.expected(key)
+    o = oracle.OracleModel.from_dict(nam, fast_tanh=fast)
+    assert (want["in_channels"], want["out_channels"], want["prewarm_samples"]) == (
+        o.in_channels, o.out_channels, o.prewarm_samples), label
+    o.reset(48000.0, block)
+    x = fx.synthetic_batch(o.in_channels, n, seed=seed)
+    yo = np.concatenate([np.atleast_2d(o.process(np.ascontiguousarray(x[:, p:p + block]))) for p in range(0, n, block)],
+                        axis=1)
+    o.close()
+    err = np.max(np.abs(want["y"] - R.sample(yo)), axis=0)  # per sampled frame, over the channels
+    assert float(err.max()) <= TOL, f"{label} block at {int(np.argmax(err)) * R.STRIDE // block * block}: {err.max():.3e}"
+
+
 def test_multichannel_models():
     """in_channels / out_channels != 1 (NAM/wavenet/model.cpp:809-820,888-909; NAM/lstm.cpp:103-125): the oracle's
     reading of the channel handling against the reference build, DSP::process with channel arrays."""
-    for label, nam in _multichannel_models():
-        r = ref.ReferenceModel.from_dict(nam)
-        o = oracle.OracleModel.from_dict(nam)
-        assert (r.in_channels, r.out_channels) == (o.in_channels, o.out_channels), label
-        r.reset(48000.0, 64)
-        o.reset(48000.0, 64)
-        x = fx.synthetic_batch(r.in_channels, 640, seed=17)
-        for p in range(0, 640, 64):
-            yr = r.process_planar(x[:, p:p + 64])
-            yo = np.atleast_2d(o.process(np.ascontiguousarray(x[:, p:p + 64])))
-            err = float(np.max(np.abs(yr - yo)))
-            assert err <= TOL, f"{label} block at {p}: {err:.3e}"
-        r.close()
-        o.close()
+    for i, (label, nam) in enumerate(_multichannel_models()):
+        _planar_against_the_reference(nam, False, 640, 64, 17, f"multichannel/{i}", label)
 
 
 def _convnet(channels, dilations, batchnorm, activation, seed, in_channels=1, out_channels=1, groups=1):
@@ -193,20 +172,7 @@ CONVNETS = [
 def test_convnet(kw, fast):
     """NAM/convnet.cpp (kernel-2 dilated Conv1D -> BatchNorm -> activation blocks, linear head): the reference's own
     tests only assert isfinite (tools/test/test_convnet.cpp), so the oracle's reading is held to the reference build."""
-    nam = _convnet(**kw)
-    r = ref.ReferenceModel.from_dict(nam, fast_tanh=fast)
-    o = oracle.OracleModel.from_dict(nam, fast_tanh=fast)
-    assert (r.in_channels, r.out_channels, r.prewarm_samples) == (o.in_channels, o.out_channels, o.prewarm_samples)
-    r.reset(48000.0, 96)
-    o.reset(48000.0, 96)
-    x = fx.synthetic_batch(r.in_channels, 960, seed=23)
-    for p in range(0, 960, 96):
-        yr = r.process_planar(x[:, p:p + 96])
-        yo = np.atleast_2d(o.process(np.ascontiguousarray(x[:, p:p + 96])))
-        err = float(np.max(np.abs(yr - yo)))
-        assert err <= TOL, f"block at {p}: {err:.3e}"
-    r.close()
-    o.close()
+    _planar_against_the_reference(_convnet(**kw), fast, 960, 96, 23, f"convnet/{CONVNETS.index(kw)}/{R.regime(fast)}")
 
 
 def _slimmable_models():
@@ -249,23 +215,14 @@ def test_slimmable_wavenet_slicing(case):
     label, nam = list(_slimmable_models())[case]
     subs = nb.submodels(nam)
     assert len(subs) >= 2 and subs[-1][0] >= 1.0
-    r0 = ref.ReferenceModel.from_dict(nam)
+    want = R.expected(f"slimmable/{case}")
+    ratios = R.slimmable_ratios(subs)
+    assert np.array_equal(want["ratios"], ratios), f"{label}: the sub-model breakpoints moved: {ratios}"
     x = fx.synthetic_batch(1, 1500, seed=41)[0]
-    bps = [mv for mv, _ in subs[:-1]]
-    ratios = sorted({0.0, 1.0, *bps, *[(a + b) / 2 for a, b in zip([0.0] + bps, bps + [1.0])]})
-    for val in ratios:
-        r = ref.ReferenceModel.from_dict(nam)
-        r.reset(48000.0, 64)
-        r.set_slimmable_size(val)
-        yr = r.run(x, 64)
-        r.close()
+    for val, yr in zip(ratios, want["y"]):
         idx = next((i for i, (mv, _) in enumerate(subs) if val < mv), len(subs) - 1)
-        o = oracle.OracleModel.from_dict(subs[idx][1])
-        o.reset(48000.0, 64)
-        yo = o.run(x, 64)
-        o.close()
+        yo = R.sample(_oracle(subs[idx][1], x))
         assert _rel(float(np.max(np.abs(yr - yo))), yr) <= TOL, f"{label}: ratio {val} -> sub-model {idx}"
-    r0.close()
 
 
 @pytest.mark.parametrize("impl", ["direct", "fft", "auto"])
@@ -273,17 +230,27 @@ def test_linear_fft_and_direct_form_are_the_same_filter(impl):
     """NAM/linear.cpp:99-113,201-278: above 256 taps the reference's Linear switches ("auto") or can be told ("fft") to a
     partitioned-FFT evaluation of the same FIR.  The product runs direct form at any length (SURVEY.md 8f-4), so the two
     must agree: the reference build with each implementation against the oracle's direct form."""
+    x = fx.synthetic_batch(1, 3000, seed=5)[0]
+    want = R.sample(_oracle(linear_fir(impl), x))
+    got = R.expected(f"linear/{impl}")["y"]
+    assert float(np.max(np.abs(got - want))) <= 2e-6
+
+
+def linear_fir(impl):
+    """A 600-tap Linear model (past the reference's 256-tap switch to FFT) with the given "implementation"."""
     rng = np.random.default_rng(12)
     rf = 600
-    nam = {"version": "0.5.4", "architecture": "Linear", "sample_rate": 48000,
-           "config": {"receptive_field": rf, "bias": True, "implementation": impl},
-           "weights": [float(v) for v in rng.uniform(-0.05, 0.05, rf + 1)]}
-    x = fx.synthetic_batch(1, 3000, seed=5)[0]
-    m = oracle.OracleModel.from_dict(nam)
-    m.reset(48000.0, 64)
-    want = m.run(x, 64)
-    r = ref.ReferenceModel.from_dict(nam)
-    r.reset(48000.0, 64)
-    got = r.run(x, 64)
-    r.close()
-    assert float(np.max(np.abs(got - want))) <= 2e-6
+    return {"version": "0.5.4", "architecture": "Linear", "sample_rate": 48000,
+            "config": {"receptive_field": rf, "bias": True, "implementation": impl},
+            "weights": [float(v) for v in rng.uniform(-0.05, 0.05, rf + 1)]}
+
+
+@pytest.mark.skipif(not (ref.available() and ref.available("generic")), reason="oracle/_ref/ not built")
+def test_recorded_outputs_are_the_reference_builds():
+    """tests/golden/reference_outputs.npz is what the reference build computes: every recorded run, repeated."""
+    with np.load(R.GOLDEN) as z:
+        stored = {k: z[k] for k in z.files}
+    fresh = R.record()
+    assert sorted(fresh) == sorted(stored)
+    for key, val in fresh.items():
+        assert val.shape == stored[key].shape and float(np.max(np.abs(val - stored[key]), initial=0.0)) <= 1e-6, key

@@ -3,9 +3,7 @@
 #   build/nam_b200_bench        our own C++ tool over the C ABI
 #   build/nam_b200_multi_test   a C++ host driving several GPUs through the C ABI (nam_b200_multi_*)
 #   build/microbench            design-constant micro-benchmarks (tools/microbench.cu)
-#   build/ref_tools/{benchmodel,benchmodel_bufsize,loadmodel,render}   -- only when the reference tree is mounted: the
-#       reference's OWN tool sources, compiled UNCHANGED from where they lie, against include/NAM/*.h and
-#       libnam_b200.so.  This is the drop-in proof: nothing of the reference is copied into the repo.
+# (The reference's own tools, compiled unchanged against include/NAM/*.h, are built by `make -C oracle ref_tools`.)
 set -euo pipefail
 ROOT="$(cd "$(dirname "$0")/.." && pwd)"
 LIBDIR="$ROOT/neuralampmodelercore_b200/lib"
@@ -17,13 +15,4 @@ CXX=${CXX:-g++}
   -L"$LIBDIR" -lnam_b200 -Wl,-rpath,'$ORIGIN/../neuralampmodelercore_b200/lib'
 if command -v nvcc >/dev/null 2>&1; then
   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -o "$ROOT/build/microbench" "$ROOT/tools/microbench.cu"
-fi
-REF=${NAM_REFERENCE:-/root/reference}
-if [ -d "$REF/tools" ]; then
-  mkdir -p "$ROOT/build/ref_tools"
-  for t in benchmodel benchmodel_bufsize loadmodel render; do
-    "$CXX" -std=c++20 -O2 -I"$ROOT/include" -o "$ROOT/build/ref_tools/$t" "$REF/tools/$t.cpp" \
-      -L"$LIBDIR" -lnam_b200 -Wl,-rpath,'$ORIGIN/../../neuralampmodelercore_b200/lib'
-  done
-  echo "built reference tools unchanged against include/NAM: $(ls "$ROOT/build/ref_tools" | tr '\n' ' ')"
 fi
