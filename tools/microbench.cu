@@ -3,11 +3,15 @@
 //   2. the kernel's inner-loop pattern: one warp-uniform weight row (16 floats = 4 x LDS.128)
 //      feeding S x 8 FFMA2 (S = time steps per thread); weights from shared memory or from
 //      __constant__ memory
+//   3. `microbench packed-const`: the compiled kernel's pattern, packed FFMA2 with constant-bank weight pairs
+//      against FFMA-immediate
 // Prints one JSON object per line.  Build: nvcc -gencode arch=compute_100a,code=sm_100a -O3 -o microbench microbench.cu
 #include <cuda_runtime.h>
 
 #include <cstdio>
 #include <cstdlib>
+#include <string>
+#include <utility>
 #include <vector>
 
 #define CK(x)                                                                                                        \
@@ -124,6 +128,87 @@ __global__ void __launch_bounds__(128) inner_loop(const float4* __restrict__ w, 
     out[0] = s;
 }
 
+// 3. The compiled kernel's straight-line pattern at one frame per thread, 16 channels, over a weight image the size
+// of a1_standard's (c_weights: 896 rows of 16 floats = 56 KB), layers of 16 rows whose outputs feed the next layer's
+// inputs.
+//   PACKED = false: scalar FFMA with the weight as immediate (what wavenet_spec_kernel compiles to today).
+//   PACKED = true:  FFMA2 over output-channel pairs, input broadcast from one register, the weight pair from a uniform
+//                   register loaded from the constant bank (LDCU.128 = two pairs per load).
+constexpr int kPackedConstRows = kConstRows;
+
+__host__ __device__ constexpr float packed_const_weight(int r, int o)
+{
+  return 0.0625f + 1e-3f * ((r * 16 + o) % 97);
+}
+
+// One layer: 16 rows at compile-time offsets (every weight an immediate or a constant-bank address), then its outputs
+// become the next layer's inputs.
+template <bool PACKED, int L>
+__device__ __forceinline__ void packed_const_layer(float (&x)[16], float2 (&acc)[8])
+{
+#pragma unroll
+  for (int i = 0; i < 16; i++)
+  {
+    const int r = L * 16 + i;
+    if (PACKED)
+    {
+      const float2 xx = make_float2(x[i], x[i]);
+#pragma unroll
+      for (int q = 0; q < 4; q++)
+      {
+        const float4 w = c_weights[r * 4 + q];
+        acc[2 * q] = __ffma2_rn(xx, make_float2(w.x, w.y), acc[2 * q]);
+        acc[2 * q + 1] = __ffma2_rn(xx, make_float2(w.z, w.w), acc[2 * q + 1]);
+      }
+    }
+    else
+    {
+#pragma unroll
+      for (int q = 0; q < 8; q++)
+      {
+        acc[q].x = fmaf(x[i], packed_const_weight(r, 2 * q), acc[q].x);
+        acc[q].y = fmaf(x[i], packed_const_weight(r, 2 * q + 1), acc[q].y);
+      }
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < 8; q++)
+  {
+    x[2 * q] = acc[q].x;
+    x[2 * q + 1] = acc[q].y;
+  }
+}
+
+template <bool PACKED, int... L>
+__device__ __forceinline__ void packed_const_layers(float (&x)[16], float2 (&acc)[8], std::integer_sequence<int, L...>)
+{
+  (packed_const_layer<PACKED, L>(x, acc), ...);
+}
+
+template <bool PACKED, int MIN_CTAS>
+__global__ void __launch_bounds__(512, MIN_CTAS) packed_const(float* out, long long* cycles, int iters)
+{
+  float x[16];
+  float2 acc[8];
+#pragma unroll
+  for (int i = 0; i < 16; i++)
+    x[i] = 1e-3f * (threadIdx.x + i);
+#pragma unroll
+  for (int q = 0; q < 8; q++)
+    acc[q] = make_float2(0.f, 0.f);
+  const long long t0 = clock64();
+  for (int it = 0; it < iters; it++)
+    packed_const_layers<PACKED>(x, acc, std::make_integer_sequence<int, kPackedConstRows / 16>{});
+  if (threadIdx.x == 0 && blockIdx.x == 0)
+    cycles[0] = clock64() - t0;
+  float s = 0.f;
+#pragma unroll
+  for (int q = 0; q < 8; q++)
+    s += acc[q].x + acc[q].y;
+  if (s == 12345.678f)
+    out[0] = s;
+}
+
 static double time_ms(cudaEvent_t e0, cudaEvent_t e1)
 {
   float ms;
@@ -132,7 +217,56 @@ static double time_ms(cudaEvent_t e0, cudaEvent_t e1)
   return ms;
 }
 
-int main()
+// `microbench packed-const`: FMA/clk/SM of the packed constant-bank form against scalar FFMA-immediate, 16/32/64
+// warps per SM, 512-thread CTAs, one wave.  Per clock is given both at the attribute's max clock (comparable with the
+// other tests) and at the SM clock block 0 counted during the run.
+static void run_packed_const(int sms, int clock_khz, float* d, cudaEvent_t e0, cudaEvent_t e1)
+{
+  std::vector<float4> hw(kPackedConstRows * 4);
+  for (int r = 0; r < kPackedConstRows; r++)
+    for (int q = 0; q < 4; q++)
+      hw[r * 4 + q] = make_float4(packed_const_weight(r, 4 * q), packed_const_weight(r, 4 * q + 1),
+                                  packed_const_weight(r, 4 * q + 2),
+                                  packed_const_weight(r, 4 * q + 3));
+  CK(cudaMemcpyToSymbol(c_weights, hw.data(), sizeof(float4) * hw.size()));
+  long long* dcyc;
+  CK(cudaMalloc(&dcyc, sizeof(long long)));
+  const int iters = 256;
+  for (int warps_per_sm : {16, 32, 64})
+    for (int packed = 0; packed < 2; packed++)
+    {
+      const int ctas_per_sm = warps_per_sm / 16, blocks = sms * ctas_per_sm;
+      auto kern = packed ? (warps_per_sm == 64 ? packed_const<true, 4> : packed_const<true, 2>)
+                         : (warps_per_sm == 64 ? packed_const<false, 4> : packed_const<false, 2>);
+      cudaFuncAttributes fa;
+      CK(cudaFuncGetAttributes(&fa, kern));
+      double best = 1e30;
+      long long cyc = 0, hcyc = 0;
+      for (int rep = 0; rep < 5; rep++) // rep 0 warms up
+      {
+        CK(cudaEventRecord(e0));
+        kern<<<blocks, 512>>>(d, dcyc, iters);
+        CK(cudaEventRecord(e1));
+        const double ms = time_ms(e0, e1);
+        CK(cudaMemcpy(&hcyc, dcyc, sizeof(hcyc), cudaMemcpyDeviceToHost));
+        if (rep > 0 && ms < best)
+        {
+          best = ms;
+          cyc = hcyc;
+        }
+      }
+      const double fma_per_sm = 16.0 * kPackedConstRows * iters * 512.0 * ctas_per_sm;
+      printf("{\"test\": \"packed_const\", \"form\": \"%s\", \"warps_per_sm\": %d, \"ms\": %.3f, "
+             "\"sm_clock_mhz\": %.0f, \"fma_per_clk_per_sm_at_max_clock\": %.1f, \"fma_per_clk_per_sm\": %.1f, "
+             "\"regs\": %d, \"spill_bytes\": %d}\n",
+             packed ? "FFMA2 x-broadcast, UR weight pair (LDCU.128)" : "FFMA immediate", warps_per_sm, best,
+             cyc / (best * 1e3), fma_per_sm / (best * 1e-3) / (clock_khz * 1e3), fma_per_sm / cyc, fa.numRegs,
+             (int)fa.localSizeBytes);
+    }
+  CK(cudaFree(dcyc));
+}
+
+int main(int argc, char** argv)
 {
   cudaDeviceProp prop;
   CK(cudaGetDeviceProperties(&prop, 0));
@@ -145,6 +279,11 @@ int main()
   cudaEvent_t e0, e1;
   CK(cudaEventCreate(&e0));
   CK(cudaEventCreate(&e1));
+  if (argc > 1 && std::string(argv[1]) == "packed-const")
+  {
+    run_packed_const(sms, clock_khz, d, e0, e1);
+    return 0;
+  }
 
   // 1. raw FMA peaks vs resident warps per SM
   for (int packed = 0; packed < 2; packed++)
